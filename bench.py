@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- contract benchmark of the 4K-NeRF ray-march hot path on B200.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Metric (BASELINE.json): rays/s of march + interp + MLP + composite.
@@ -17,6 +17,12 @@ rank marches its band and the packed bands are all-gathered with NCCL ("scaling"
 
 Timing: CUDA events on the launching stream around exactly K steps, barrier + synchronize on both
 sides, max over ranks.  Inputs per step (439 MB of rays + 213 MB of grids) exceed the 126 MB L2.
+
+`--dump-outputs DIR`: after the timed steps, the per-ray results of the last one (rgb_marched, depth,
+alphainv_last: what render_rays hands its caller) at a fixed, seeded sample of 2^20 rays, and the
+sampled ray indices, as DIR/<name>.npy (28 MB in all).  The scene and the rays are seeded, so two
+builds run with the same arguments can be compared output for output.  Geometry (depth, alphainv_last)
+repeats bit for bit from run to run; rgb_marched may differ in the last bit (1.8e-7 measured on a B200 at its 1000 W power limit).
 
 `--impl reference`: the reference has NO CPU implementation of this path (every op is CUDA-only,
 lib/cuda/render_utils.cpp:46-48) and cannot be imported here, so the arm times the oracle port
@@ -67,7 +73,12 @@ def parse_args():
     ap.add_argument('--regime', default='fog', choices=['fog', 'shell'])
     ap.add_argument('--no-extra', action='store_true', help='skip the secondary measurements')
     ap.add_argument('--no-cpu-baseline', action='store_true')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the last timed step\'s per-ray results (seeded sample of rays) as DIR/<name>.npy')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -239,6 +250,16 @@ def run_reference_arm(args, rank):
     print(json.dumps(line), flush=True)
 
 
+def dump_outputs(out, n_rays, path, n_sample=1 << 20):
+    """`--dump-outputs`: the frame's per-ray results at a fixed, seeded sample of rays, as float32 / float64 .npy."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    idx = torch.randperm(n_rays, generator=torch.Generator().manual_seed(0))[:n_sample].sort().values
+    np.save(os.path.join(path, 'ray_index.npy'), idx.double().numpy())
+    for k in ('rgb_marched', 'depth', 'alphainv_last'):
+        np.save(os.path.join(path, k + '.npy'), out[k][idx.to(out[k].device)].float().cpu().numpy())
+
+
 def workload_config(args, n_gpus):
     return {
         'workload': 'north-star target: BASELINE configs[1] model (DirectVoxGO 160^3, k0 12 ch, rgbnet 39-128-128-3, '
@@ -380,6 +401,8 @@ def main():
     clocks = sampler.summary(t_wall0, t_wall1) if rank == 0 else None
     ms_per_step = ms_total / max(args.steps, 1)
     value = (H * W) / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(full if world > 1 else frame.out, H * W, args.dump_outputs)
 
     # ---- e2e: the public API with HOST buffers (pinned rays in, host results out), every step ----
     e2e = None

@@ -1,6 +1,7 @@
 """GPU parity of the contracted-space front-end (DirectContractedVoxGO, SURVEY.md section 8(f-3)):
 fused kernel vs the CPU oracle (oracle/pipeline.dcvgo_forward) and vs the same forward structure
-running on the reference's own CUDA kernels (oracle/_ref: render_utils_cuda + ub360_utils_cuda)."""
+running on the reference's own CUDA kernels (render_utils_cuda + ub360_utils_cuda, replayed from their
+stored results: tests/ref_calls.py)."""
 import os
 
 import pytest
@@ -8,15 +9,16 @@ import torch
 
 from helpers import make_state, model_from_state, rays_for, compare
 from oracle import ops, pipeline
+from ref_calls import RefCalls
 
 pytestmark = pytest.mark.gpu
 
 
-@pytest.fixture(scope='module')
-def ref_ops(cuda_device):
-    if not os.path.exists(os.path.join(os.path.dirname(ops.ref_ext_path()), 'ub360_utils_cuda.so')):
-        pytest.skip('oracle/_ref/ub360_utils_cuda.so not built (python oracle/build_ref.py where /root/reference exists)')
-    return ops.RefExtOps()
+@pytest.fixture
+def ref_ops(request, cuda_device):
+    rc = RefCalls.for_test(request)
+    yield rc.ops()
+    rc.finish()
 
 
 def test_cumdist_thres_oracle_vs_reference_kernel(ref_ops, cuda_device):

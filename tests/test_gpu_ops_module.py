@@ -1,21 +1,21 @@
 """GPU: k4nerf.render_utils_cuda (the 13-function op-level drop-in, csrc/k4_ops.cu) against the
-REFERENCE'S OWN compiled extension (oracle/_ref/render_utils_cuda.so): every output bit-identical."""
-import os
-
+REFERENCE'S OWN compiled extension (replayed from its stored results, tests/ref_calls.py): every output
+bit-identical."""
 import pytest
 import torch
 
-from oracle import ops, scenes
+from oracle import scenes
+from ref_calls import RefCalls
 
 pytestmark = pytest.mark.gpu
 
 
-@pytest.fixture(scope='module')
-def mods(cuda_device):
-    if not os.path.exists(ops.ref_ext_path()):
-        pytest.skip('oracle/_ref/render_utils_cuda.so not built')
+@pytest.fixture
+def mods(request, cuda_device):
     from k4nerf import render_utils_cuda as ours
-    return ours, ops.load_ref_ext()
+    rc = RefCalls.for_test(request)
+    yield ours, rc.module('render_utils_cuda')
+    rc.finish()
 
 
 def _rays(n, dev, seed=0):
@@ -52,7 +52,7 @@ def test_sampling_ops_bit_exact(mods, cuda_device):
     mn2, mx2 = torch.tensor([-1.5, -1.67, -1.], device=dev), torch.tensor([1.5, 1.67, 1.], device=dev)
     for name, a, b in zip(('ndc_pts', 'ndc_mask'), ours.sample_ndc_pts_on_rays(o, d, mn2, mx2, 64), ref.sample_ndc_pts_on_rays(o, d, mn2, mx2, 64)):
         _eq(a, b, name)
-    tm = (torch.rand(ro.shape[0], device=dev) * 2 + 1).contiguous()
+    tm = (torch.rand(ro.shape[0], generator=torch.Generator().manual_seed(1)) * 2 + 1).to(dev).contiguous()
     _eq(ours.sample_bg_pts_on_rays(ro, rd, tm, 0.5, 32), ref.sample_bg_pts_on_rays(ro, rd, tm, 0.5, 32), 'bg_pts')
 
 

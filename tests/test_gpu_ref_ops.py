@@ -1,26 +1,25 @@
 """GPU: pin the oracle against the REFERENCE'S OWN KERNELS.
 
-oracle/_ref/render_utils_cuda.so is the reference extension (lib/cuda/render_utils*.{cpp,cu})
-compiled from /root/reference by oracle/build_ref.py.  Here every forward op of the C restatement
-(oracle/render_utils_ref.c) is compared with it on seeded inputs, and the whole reference pipeline
-run on the reference kernels (oracle/pipeline.py + RefExtOps) is compared with the fused kernel.
+The reference extension (lib/cuda/render_utils*.{cpp,cu}) is replayed from the digests of what it
+returned (tests/ref_calls.py).  Here every forward op of the C restatement (oracle/render_utils_ref.c)
+is compared with it on seeded inputs, and the whole reference pipeline run on the reference kernels
+(oracle/pipeline.py + the reference ops) is compared with the fused kernel.
 """
-import os
-
 import pytest
 import torch
 
 from oracle import ops, pipeline, scenes
 from helpers import compare, make_state, model_from_state, rays_for
+from ref_calls import RefCalls
 
 pytestmark = pytest.mark.gpu
 
 
-@pytest.fixture(scope='module')
-def ref_ops(cuda_device):
-    if not os.path.exists(ops.ref_ext_path()):
-        pytest.skip('oracle/_ref/render_utils_cuda.so not built (needs /root/reference at build time)')
-    return ops.RefExtOps()
+@pytest.fixture
+def ref_ops(request, cuda_device):
+    rc = RefCalls.for_test(request)
+    yield rc.ops()
+    rc.finish()
 
 
 def _rays(n, seed=0):

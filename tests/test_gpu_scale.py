@@ -4,7 +4,7 @@ The small-scene tests (test_gpu_marcher.py, test_gpu_ref_ops.py) pin the arithme
 configurations BASELINE.json names -- 160^3 grids at 1008x756, the [384,384,256] LLFF MPI model, a
 >1 M-ray band of the 4032x3024 frame, the 160^3 contracted model -- through the reference's own
 forward structure in the reference's 8192-ray chunks (run_sr.py:121-124) on the REFERENCE'S OWN CUDA
-KERNELS + ATen fp32 (oracle/pipeline.py + RefExtOps = oracle/_ref/render_utils_cuda.so, TF32 off),
+KERNELS + ATen fp32 (oracle/pipeline.py + the reference ops replayed by tests/ref_calls.py, TF32 off),
 against ONE fused launch of the tcgen05 marcher (mode `ws`, what `auto` resolves to for these shapes).
 These sizes fill all 148 persistent CTAs with many tiles each, ragged last batches included.
 
@@ -18,27 +18,28 @@ import os
 import pytest
 import torch
 
-from oracle import ops, pipeline, scenes
+from oracle import pipeline, scenes
 from helpers import compare, make_state, model_from_state, ref_forward_chunked
+from ref_calls import RefCalls
 
 pytestmark = pytest.mark.gpu
 
 
-@pytest.fixture(scope='module')
-def ref_ops(cuda_device):
-    if not os.path.exists(ops.ref_ext_path()):
-        pytest.skip('oracle/_ref/render_utils_cuda.so not built (needs /root/reference at build time)')
+@pytest.fixture
+def ref_ops(request, cuda_device):
     torch.backends.cuda.matmul.allow_tf32 = False
     torch.backends.cudnn.allow_tf32 = False
-    return ops.RefExtOps()
+    rc = RefCalls.for_test(request)
+    yield rc.ops()
+    rc.finish()
 
 
 def _log(rec):
-    """One JSON line per case into gpurun_out/ (copied to profiles/ as the parity evidence of the round)."""
+    """One JSON line per case appended to the file K4_SCALE_PARITY_LOG names, if it is set (the parity evidence)."""
     import json
-    d = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'gpurun_out')
-    if os.path.isdir(d):
-        with open(os.path.join(d, 'scale_parity.jsonl'), 'a') as f:
+    path = os.environ.get('K4_SCALE_PARITY_LOG')
+    if path:
+        with open(path, 'a') as f:
             f.write(json.dumps(rec) + '\n')
 
 
@@ -119,8 +120,6 @@ def test_cfgB_mpi_384x384x256_at_1008x756(ref_ops, cuda_device, regime):
 
 def test_cfgC_contracted_160(ref_ops, cuda_device):
     """DirectContractedVoxGO at 160^3 (the fine-stage grid size), 504x378, camera inside the unit cube."""
-    if not os.path.exists(os.path.join(os.path.dirname(ops.ref_ext_path()), 'ub360_utils_cuda.so')):
-        pytest.skip('oracle/_ref/ub360_utils_cuda.so not built')
     st = make_state('cfgC', res=160, regime='fog')
     rays = scenes.blender_rays(378, 504, radius=0.6)
     # contracted sampling: sample positions go through torch's norm / division chain (lib/dcvgo.py:237-262); at this size

@@ -1,27 +1,26 @@
 """GPU: the training-side forward (k4nerf/train_forward.py, SURVEY.md section 8 f-2).
 
 (i) values: the per-sample lists and per-ray outputs against the oracle pipeline running on the
-reference's own kernels (oracle/_ref) on the same device; (ii) gradients: against a float64 pure-torch
+reference's own kernels (replayed from their stored results, tests/ref_calls.py) on the same device; (ii) gradients: against a float64 pure-torch
 restatement of alpha / transmittance / compositing with autograd (no custom backward anywhere);
 (iii) a few MaskedAdam steps reduce the loss."""
-import os
-
 import pytest
 import torch
 
 import k4nerf
 from k4nerf import train_forward
 from helpers import make_state, model_from_state, rays_for
-from oracle import ops, pipeline
+from oracle import pipeline
+from ref_calls import RefCalls
 
 pytestmark = pytest.mark.gpu
 
 
-@pytest.fixture(scope='module')
-def ref_ops(cuda_device):
-    if not os.path.exists(os.path.join(os.path.dirname(ops.ref_ext_path()), 'ub360_utils_cuda.so')):
-        pytest.skip('oracle/_ref not built')
-    return ops.RefExtOps()
+@pytest.fixture
+def ref_ops(request, cuda_device):
+    rc = RefCalls.for_test(request)
+    yield rc.ops()
+    rc.finish()
 
 
 def _state(name, regime):

@@ -1,11 +1,9 @@
 """GPU: grid-maintenance and optimiser kernels (SURVEY.md section 8 f-4, csrc/k4_train.cu).
 
 total_variation_add_grad and the three Adam updates are compared BIT FOR BIT with the reference's own
-extensions (oracle/_ref/total_variation_cuda.so, adam_upd_cuda.so, built by oracle/build_ref.py);
+extensions (total_variation_cuda, adam_upd_cuda; replayed from their stored results, tests/ref_calls.py);
 update_occupancy_cache / scale_volume_grid are compared with the reference's torch composition
 (F.grid_sample + Raw2Alpha formula + F.max_pool3d, F.interpolate) run on the same GPU."""
-import os
-
 import pytest
 import torch
 import torch.nn.functional as F
@@ -14,21 +12,22 @@ import k4nerf
 from k4nerf import adam_upd_cuda, total_variation_cuda
 from helpers import make_state, model_from_state
 from oracle import ops
+from ref_calls import RefCalls
 
 pytestmark = pytest.mark.gpu
 
 
-def _ref(name):
-    path = os.path.join(os.path.dirname(ops.ref_ext_path()), name + '.so')
-    if not os.path.exists(path):
-        pytest.skip(f'oracle/_ref/{name}.so not built (python oracle/build_ref.py where /root/reference exists)')
-    return ops.load_ref_ext(name)
+@pytest.fixture
+def ref_calls(request, cuda_device):
+    rc = RefCalls.for_test(request)
+    yield rc
+    rc.finish()
 
 
 @pytest.mark.parametrize('shape', [(1, 1, 17, 9, 33), (1, 12, 20, 24, 16), (1, 3, 1, 5, 2)])
 @pytest.mark.parametrize('dense', [True, False])
-def test_total_variation_add_grad_bit_exact(cuda_device, shape, dense):
-    ref = _ref('total_variation_cuda')
+def test_total_variation_add_grad_bit_exact(cuda_device, ref_calls, shape, dense):
+    ref = ref_calls.module('total_variation_cuda')
     g = torch.Generator().manual_seed(3)
     param = (torch.randn(shape, generator=g) * 1.5).to(cuda_device)
     grad = torch.randn(shape, generator=g)
@@ -46,8 +45,8 @@ def test_total_variation_add_grad_bit_exact(cuda_device, shape, dense):
 
 @pytest.mark.parametrize('n', [4096 * 3, 1001])               # float4 path and the scalar tail path
 @pytest.mark.parametrize('variant', ['plain', 'masked', 'perlr'])
-def test_adam_updates_bit_exact(cuda_device, n, variant):
-    ref = _ref('adam_upd_cuda')
+def test_adam_updates_bit_exact(cuda_device, ref_calls, n, variant):
+    ref = ref_calls.module('adam_upd_cuda')
     g = torch.Generator().manual_seed(7)
     mk = lambda s=1.0: (torch.randn(n, generator=g) * s).to(cuda_device)
     p0, m0, v0 = mk(), mk(0.1), (mk(0.1) ** 2)
